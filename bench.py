@@ -15,6 +15,8 @@ exactly K timed steps:
            on a bounded sample of the same workload.
 --impl reference times the reference's CPU path (the oracle port; the Java reference cannot run here:
 no JVM) on the host cores with the same step definition.
+--dump-outputs DIR writes the state the timed network holds after its last step (what a caller reads back) as .npy files,
+so that two builds can be compared output for output on identical, seeded inputs.
 """
 import argparse
 import json
@@ -133,6 +135,52 @@ def state_digests(p, lo=None, hi=None):
     for k, v in p.level_scalars().items():
         out["level_" + k] = dg(v)
     return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def gsf_outputs(p):
+    """What a caller reads back after runMs on a GSFSignature object (engine, shard or oracle): the per-node scalars, the 5
+    node counters and a fixed, seeded sample of verifiedSignatures rows (the whole bitmap is N^2/8 bytes), each row as its
+    32-bit words so that float64 holds them exactly."""
+    import numpy as np
+
+    q = getattr(p, "local", p)
+    net = q if hasattr(q, "counters") else q.network()
+    out = {"scalar_" + k: v for k, v in q.scalars().items()}
+    out["counters"] = net.counters()
+    ver = q.verified()
+    rows = max(1, min(256, len(ver), (16 << 20) // (ver.shape[1] * 2 * 8)))
+    idx = np.sort(np.random.default_rng(0).choice(len(ver), rows, replace=False))
+    out["verified_sample_rows"] = idx
+    out["verified_sample"] = np.ascontiguousarray(ver[idx]).view(np.uint32)
+    return out
+
+
+def casper_outputs(p):
+    """What a caller reads back after runMs on a CasperIMD object (engine, shard or oracle): node state (the 64-bit
+    attestation hash as its 32-bit words) and the 5 node counters."""
+    import numpy as np
+
+    q = getattr(p, "local", p)
+    net = q if hasattr(q, "counters") else q.network()
+    out = {"node_" + k: v for k, v in q.node_state().items()}
+    out["node_att_hash"] = out["node_att_hash"].view(np.uint32).reshape(-1, 2)
+    out["counters"] = net.counters()
+    return out
+
+
+def dump_outputs(d, arrays):
+    """--dump-outputs: each array as <d>/<name>.npy in float64 (exact for the engine's integer state)."""
+    import numpy as np
+
+    total = sum(a.size * 8 for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), np.asarray(a, np.float64))
 
 
 def event_counts(st0, st1):
@@ -268,6 +316,8 @@ def run_reference(args):
     del w
     wall = o.run_timed(step_ms, args.steps)
     val = args.steps * step_ms / wall
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, gsf_outputs(o))
     line = {"impl": "reference", "metric": metric_name(args.nodes), "value": val, "unit": "simulated-ms/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000 * wall / args.steps, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "u64 bitmaps / int32", "data": "synthetic",
@@ -316,6 +366,8 @@ def run_casper_reference(args):
     d0 = o.deliveries()
     wall = o.run_timed(8000 * K, 8000)
     val = 8000 * K / wall
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, casper_outputs(o))
     print(json.dumps({"impl": "reference", "metric": "simulated-ms/sec, CasperIMD 16,390 nodes", "value": val, "unit": "simulated-ms/s",
                       "n_gpus": args.gpus, "steps": K, "warmup": W, "ms_per_step": 1000 * wall / K, "higher_is_better": True,
                       "scaling": "weak", "vs_baseline": None, "dtype": "u64 bitmaps / int32", "data": "synthetic",
@@ -371,6 +423,8 @@ def run_casper(args, rank, world, local, dist, barrier, max_over_ranks, sum_over
     st1 = net.stats()
     heads_end = p.heads()
     nblocks = len(p.blocks()["height"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, casper_outputs(p))
     del p, net
     # pass 2: end to end with the read-backs a caller makes after every slot (heads + the five node counters)
     p = make()
@@ -489,6 +543,9 @@ def main():
     ap.add_argument("--weak-nodes-per-gpu", type=int, default=32768)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed network holds after its last step as DIR/<name>.npy "
+                         "(float64; with several ranks, rank 0's network or shard)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -571,6 +628,8 @@ def main():
     launches = st1["kernel_launches"] - st0["kernel_launches"]
     card_end = p.scalars()["card"]
     done = not p.continue_if()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gsf_outputs(p))
     dev_ms = max_over_ranks(dev_ms)
     ev_all = {k: int(total(v)) for k, v in ev.items()} if sharded else ev
     launches_all = int(total(launches)) if sharded else launches
